@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (ours; under torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K --warmup W   (reference arm: CPU oracle)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (also writes the last timed step's output to DIR)
 
 A "step" is one forward of ``LKA_Attention3d_deform`` (proj_1 -> GELU -> dw5^3 -> dw7^3 dil3 ->
 conv_offset -> deformable 3^3 conv -> conv1 -> gate -> proj_2 -> +shortcut) over one batch of synthetic
@@ -20,6 +21,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -119,6 +121,23 @@ def emit(obj):
     line = (json.dumps(obj) + "\n").encode()
     sys.stdout.flush()
     os.write(_REAL_STDOUT if _REAL_STDOUT is not None else 1, line)
+
+
+DUMP_SAMPLE = 1 << 22   # elements kept of an output larger than this (16 MB in float32)
+
+
+def dump_outputs(out_dir, **outputs):
+    """--dump-outputs: every output as <out_dir>/<name>.npy, float32, flattened.  An output of more than DUMP_SAMPLE elements is
+    written as the elements at DUMP_SAMPLE sorted positions drawn from a generator seeded with 0: the same positions in every
+    run, so two builds run with the same arguments can be compared element by element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach().reshape(-1)
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def _time_call(fn, iters=20, warm=5, reps=3):
@@ -338,7 +357,13 @@ def main():
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="c4net: launch the 21 block calls eagerly instead of replaying one CUDA graph")
     ap.add_argument("--no-profile-pass", action="store_true", help="skip the per-kernel event pass (tools/measure_traffic.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output of the last timed step to DIR/y.npy (float32; a seeded "
+                    f"sample of {DUMP_SAMPLE} of its elements, see dump_outputs); rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "headline"):
+        ap.error("--dump-outputs applies to the headline workload of --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     quiet_stdout()
@@ -400,6 +425,8 @@ def main():
         clocks = sampler.stop() if rank == 0 else None
         from deformablelka_b200.dist import max_over_ranks
         ms_total = max_over_ranks(ms, dev)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, y=y)     # y: the block output [B, N, C] of the last timed step
 
         # per-kernel durations over the same K steps (CUDA events on the launch stream, inside the library)
         prof = {}

@@ -3,6 +3,8 @@ include/dlka.h declares; the host modules keep the reference's state_dict keys; 
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 import torch
@@ -77,14 +79,15 @@ def test_backward_argument_checks_mirror_reference():
 
 
 def test_compute_entry_without_device_returns_no_device_or_runs():
-    import deformablelka_b200 as d
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    L = d._lib.lib
-    buf = (ctypes.c_float * 16)()
-    st = L.dlka_deform_conv3d_sample_indices(ctypes.addressof(buf), ctypes.addressof(buf), ctypes.addressof(buf),
-                                             1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 0, 0, 0, 1, 1, 1, 1, None)
-    assert st == -4  # DLKA_ERR_NO_DEVICE: no CPU path exists
+    # in a child process that sees no CUDA device, so that a machine with a GPU checks the same thing
+    code = ("import ctypes, deformablelka_b200 as d\n"
+            "buf = (ctypes.c_float * 16)()\n"
+            "print(d._lib.lib.dlka_deform_conv3d_sample_indices(ctypes.addressof(buf), ctypes.addressof(buf), ctypes.addressof(buf),"
+            " 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 0, 0, 0, 1, 1, 1, 1, None))\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr
+    assert r.stdout.split()[-1] == "-4"  # DLKA_ERR_NO_DEVICE: no CPU path exists
 
 
 def test_state_dict_keys_match_reference_and_oracle(oracle):

@@ -2,8 +2,10 @@
 ``D3D`` and driven with the reference's own calling sequence (3D/dcn/functions/deform_conv_func.py:15-56, restated in
 ``_RefDeformConvFunction`` below -- argument order, the kernel-size / stride / padding / dilation unpacking and the order of the
 four returned gradients are what that file does with the compiled extension)."""
+import importlib
 import importlib.util
 import inspect
+import json
 import os
 import sys
 
@@ -13,7 +15,7 @@ from torch.autograd import Function
 from torch.autograd.function import once_differentiable
 from torch.nn.modules.utils import _triple
 
-from conftest import ROOT
+from conftest import GOLDEN, ROOT
 
 SHIM = os.path.join(ROOT, "deformablelka_b200", "compat", "D3D.py")
 
@@ -38,21 +40,22 @@ def test_shim_exports_the_reference_signatures(D3D):
 
 
 def test_reference_function_source_calls_match_the_shim(D3D):
-    """When the reference tree is present (build container), its deform_conv_func.py is imported UNMODIFIED with the shim as
-    ``D3D``: the import succeeds and the Function's forward / backward reference exactly the two shim entry points."""
-    ref = "/root/reference/3D/dcn/functions/deform_conv_func.py"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not present on this box")
+    """The reference's deform_conv_func.py as recorded in tests/golden/ref3d_deform_conv_func.json (make_golden_shim.py): with
+    the shim as ``D3D`` every import it makes resolves, and its Function's forward / backward call exactly the two shim entry
+    points, each with as many positional arguments as the shim function takes."""
+    rec = json.load(open(os.path.join(GOLDEN, "ref3d_deform_conv_func.json")))
+    assert ["D3D", None] in rec["imports"]
     sys.modules["D3D"] = D3D
     try:
-        spec = importlib.util.spec_from_file_location("_ref_deform_conv_func", ref)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        assert mod.D3D is D3D and hasattr(mod.DeformConvFunction, "apply")
-        src = open(ref).read()
-        assert "D3D.deform_conv_forward(" in src and "D3D.deform_conv_backward(" in src
+        for module, name in rec["imports"]:
+            mod = importlib.import_module(module)
+            assert name is None or hasattr(mod, name), (module, name)
     finally:
         sys.modules.pop("D3D", None)
+    assert [(c["caller"], c["function"]) for c in rec["d3d_calls"]] == [
+        ("DeformConvFunction.forward", "deform_conv_forward"), ("DeformConvFunction.backward", "deform_conv_backward")]
+    for c in rec["d3d_calls"]:
+        assert len(inspect.signature(getattr(D3D, c["function"])).parameters) == c["positional_args"], c
 
 
 def _make_ref_function(D3D):
